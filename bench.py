@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N ...            # the reference algorithm on the host CPU
+    python bench.py ... --dump-outputs DIR                   # also write the last timed step's pixels as DIR/*.npy
 
 A "step" is one pass of the hot path (Multiply.forward, eval) over one batch of synthetic rays:
 BASELINE.json configs[1] = 2-person synthetic SMPL scene, 4096 rays x 128 samples (S/E/X = 128/256/64),
@@ -154,10 +155,12 @@ def run_reference(args, rank, world):
     times = []
     for i in range(args.warmup + args.steps):
         t = time.time()
-        port.multiply_forward(sc, sub, hits)
+        o = port.multiply_forward(sc, sub, hits)
         dt = time.time() - t
         if i >= args.warmup:
             times.append(dt)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, host_copy(o))
     tot = sum(times)
     val = n_sample * len(times) / tot
     line = {"impl": "reference", "metric": "rays/sec", "value": val, "unit": "rays/s", "n_gpus": args.gpus,
@@ -212,6 +215,19 @@ class Timer:
 
 def linf(a, b):
     return float((a.double().cpu() - b.double().cpu()).abs().max())
+
+
+def host_copy(out):
+    """float32 host copies of the pixel outputs (parallel.PIXEL_KEYS) of one step."""
+    from multiply_b200 import parallel
+    return {k: out[k].detach().float().cpu().numpy() for k in parallel.PIXEL_KEYS}
+
+
+def dump_outputs(path, arrays):
+    """--dump-outputs: one DIR/<name>.npy per output array, so that two builds can be compared output for output."""
+    os.makedirs(path, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(path, k + ".npy"), a)
 
 
 def extras_strong(timer, dev, rank, world, steps):
@@ -396,6 +412,8 @@ def main():
     ap.add_argument("--no-extras", action="store_true")
     ap.add_argument("--precision", default="parity", choices=["parity", "colour1", "throughput"],
                     help="tcgen05 precision mode of the main measurement (default parity: RGB/SDF within 1e-4)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the pixel outputs of the last timed step as DIR/<name>.npy (float32; rank 0, whole frame)")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -446,6 +464,10 @@ def main():
     clocks = ClockSampler(local)
     clocks.start()
     ms_value, launches = timer.run(step_resident, args.steps, args.warmup)
+    # the later passes below render into the same buffers: keep what the last timed step returned
+    last_step = None
+    if args.dump_outputs and rank == 0:
+        last_step = host_copy(parallel.PixelBuffer.frame(gathered, world, R, PERSONS) if world > 1 else buf.views)
     with torch.no_grad():
         ms_e2e, launches_e2e = timer.run(step_e2e, args.steps, args.warmup)
     model._renderer.check_status()
@@ -638,6 +660,8 @@ def main():
         extras["cuda_graph"] = graph_rec
         line["parity"] = parity
         line["extras"] = extras
+        if last_step is not None:
+            dump_outputs(args.dump_outputs, last_step)
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()

@@ -6,6 +6,7 @@ import os
 import subprocess
 import sys
 
+import numpy as np
 import pytest
 import torch
 
@@ -31,6 +32,37 @@ def test_reference_arm_line():
     e = line["e2e"]
     assert e["value"] == line["value"] and e["unit"] == line["unit"]
     assert e["h2d_bytes_per_step"] == 0 and e["d2h_bytes_per_step"] == 0
+
+
+def _dumped(d, R):
+    shapes = {"rgb_values": (R, 3), "fg_rgb_values": (R, 3), "normal_values": (R, 3), "acc_map": (R,),
+              "acc_person_list": (R, 2)}
+    assert sorted(os.listdir(d)) == sorted(k + ".npy" for k in shapes)
+    out = {k: np.load(os.path.join(d, k + ".npy")) for k in shapes}
+    for k, a in out.items():
+        assert a.dtype == np.float32 and a.shape == shapes[k] and np.isfinite(a).all(), k
+    return out
+
+
+def test_reference_arm_dump_outputs(tmp_path):
+    p = _run(["--impl", "reference", "--steps", "1", "--warmup", "0", "--dump-outputs", str(tmp_path / "out")])
+    assert p.returncode == 0, p.stderr[-2000:]
+    _dumped(tmp_path / "out", 128)
+
+
+@pytest.mark.gpu
+def test_product_arm_dump_outputs_repeat(tmp_path):
+    """Same arguments, same inputs: two runs of the timed path dump the same pixels."""
+    args = ["--steps", "2", "--warmup", "0", "--no-extras", "--no-cpu-baseline", "--dump-outputs"]
+    runs = []
+    for i in range(2):
+        d = str(tmp_path / ("run%d" % i))
+        p = _run(args + [d])
+        assert p.returncode == 0, p.stderr[-2000:]
+        assert json.loads(p.stdout.strip().splitlines()[-1])["steps"] == 2
+        runs.append(_dumped(d, 4096))
+    for k in runs[0]:
+        assert np.array_equal(runs[0][k], runs[1][k]), k
 
 
 @pytest.mark.skipif(torch.cuda.is_available(), reason="only meaningful on a box without a GPU")
